@@ -5,6 +5,7 @@
 //   warp 1        MMA issuer (one thread):  S_i = Q_i K_j^T   (tcgen05.mma SS, fp32 accumulate, 128 x BC into TMEM)
 //                                            O_i += P_ij V_j   (tcgen05.mma TS: P read from TMEM, V MN-major smem)
 //   warp 2        TMEM allocator
+//   warp 3        masked build with seqlens_k only: zeroes the V rows past the length in the last KV tile
 //   warps 4..7    softmax warpgroup for Q tile 0, one thread per query row: tcgen05.ld the S row, online softmax
 //   warps 8..11   softmax warpgroup for Q tile 1       (row max / exp2 / row sum in fp32 registers), P written as
 //                 fp16 into its OWN TMEM columns with tcgen05.st; O is rescaled in TMEM only when the row max grew
@@ -94,6 +95,31 @@ struct Fa2Mask {
   int causal = 0;
 };
 
+// Zeroes keys [valid, BC) of the V tile at shared address vt, by the 32 lanes t of one warp, and makes the zeros visible
+// to the tensor core (the caller's next mbarrier arrive orders them before the MMA).
+template <class Cfg>
+__device__ __forceinline__ void fa2_zero_v_keys(uint32_t vt, int valid, int t) {
+  constexpr int D = Cfg::D, BC = Cfg::BC, ROWB = Cfg::ROWB;
+  if constexpr (Cfg::V_DN) {
+    // [D rows x 64 keys] boxes, 128B swizzle: the 8-key piece g of row d sits in 16-byte slot (g % 8) ^ (d % 8)
+    for (int u = (valid / 8) * D + t; u < (BC / 8) * D; u += 32) {
+      const int g = u / D, d = u % D, key0 = g * 8;
+      const uint32_t addr = vt + (g / 8) * (D * 128) + d * 128 + (((g % 8) ^ (d % 8)) << 4);
+      if (key0 >= valid) {
+        st_shared_v4(addr, 0u, 0u, 0u, 0u);
+      } else {
+        for (int e = valid - key0; e < 8; ++e) st_shared_u16(addr + 2 * e, 0);
+      }
+    }
+  } else {
+    // a key is one ROWB-byte row of every CW-wide chunk; the swizzle only permutes 16-byte pieces inside a row
+    for (int u = valid * (ROWB / 16) + t; u < BC * (ROWB / 16); u += 32)
+#pragma unroll
+      for (int c = 0; c < Cfg::NCH; ++c) st_shared_v4(vt + c * Cfg::KV_CHUNK_BYTES + u * 16, 0u, 0u, 0u, 0u);
+  }
+  fence_proxy_async_smem();
+}
+
 template <class Cfg, bool TRACE, int POLY, int NP, bool MASKED = false>
 __global__ void __launch_bounds__(Cfg::THREADS, 1)
 fa2_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
@@ -123,6 +149,8 @@ fa2_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
   const uint32_t bar_p_free = bar_p_full + 64;            // 2   PV_i(j) done: P_i free, O_i stable (MMA -> softmax i)
   const uint32_t bar_o_full = bar_p_free + 16;            // 2   last PV_i done               (MMA -> softmax i)
   const uint32_t tmem_slot = bar_o_full + 16;
+  const uint32_t bar_v_zero = tmem_slot + 8;              // 1   V rows past seqlens zeroed (warp 3 -> MMA), MASKED only
+  const uint32_t bar_v_tail = tmem_slot + 16;             // 1   softmax warp 4 reached the last KV tile (-> warp 3)
   volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(base_ptr + (tmem_slot - base));
   const uint32_t smem_q = base + Cfg::BAR_BYTES;                      // 2 Q tiles
   const uint32_t smem_k = smem_q + 2 * Cfg::Q_TILE_BYTES;             // STAGES K tiles
@@ -140,6 +168,12 @@ fa2_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
   const int n_keys = (MASKED && mask.seqlens) ? min(N, max(1, mask.seqlens[bh / mask.H])) : N;  // valid keys of this batch
   const int Tk = (n_keys + BC - 1) / BC;
   const int T = causal ? min(Tk, (q0 + 256 + BC - 1) / BC) : Tk;  // KV tiles this CTA walks
+  // Key padding: the last KV tile is loaded whole, so its keys in [seqlens[b], N) are real memory that TMA does not
+  // zero-fill (it does past N).  Their P is exactly 0, but 0 * NaN / Inf in the PV product is NaN, so warp 3 zeroes those
+  // V rows in shared memory and the MMA thread issues the PV products of that tile only after it has.  Warp 3 first waits
+  // until softmax warp 4 reaches that tile: warp 4 has then seen PV_0 of tile T-3 complete, so every earlier use of the
+  // V stage has landed and the parity wait on bar_v_full below cannot be satisfied by an older phase.
+  const bool zero_v_tail = MASKED && n_keys < N && (n_keys % BC) != 0 && T == Tk;
 
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&tmQ);
@@ -155,6 +189,10 @@ fa2_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       for (int p = 0; p < 4; ++p) mbar_init(bar_p_full + 32 * i + 8 * p, 4);
       mbar_init(bar_p_free + 8 * i, 1);
       mbar_init(bar_o_full + 8 * i, 1);
+    }
+    if (MASKED) {
+      mbar_init(bar_v_zero, 32);
+      mbar_init(bar_v_tail, 1);
     }
     for (int s = 0; s < STAGES; ++s) {
       mbar_init(bar_k_full + 8 * s, 1);
@@ -267,6 +305,7 @@ fa2_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
 #pragma unroll
           for (int k = 0; k < BC / 16; ++k) {
             if (k % (BC / 16 / NP) == 0) {
+              if (k == 0 && zero_v_tail && j == Tk - 1) mbar_wait(bar_v_zero, 0);
               mbar_wait(bar_p_full + 32 * i + 8 * (k / (BC / 16 / NP)), j & 1);
               tc_fence_after();
               if (k == 0) tr(0, j, 5 + i);
@@ -368,6 +407,14 @@ fa2_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
         tr(0, j, 7);
       }
       }
+    }
+  } else if (warp == 3) {
+    if (zero_v_tail) {
+      const int j = Tk - 1, s = j % STAGES;
+      mbar_wait(bar_v_tail, 0);
+      mbar_wait(bar_v_full + 8 * s, (j / STAGES) & 1);
+      fa2_zero_v_keys<Cfg>(smem_v + s * Cfg::KV_TILE_BYTES, n_keys - j * BC, int(lane));
+      mbar_arrive(bar_v_zero);
     }
   } else if (warp >= 4) {
     // ---------------------------------------------------------------------------------- softmax + epilogue
@@ -485,6 +532,7 @@ fa2_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
     for (int j = 0; j < T; ++j) {
       uint32_t sr[BC];
       const bool tw = TRACE && lane == 0 && q == 0;
+      if (zero_v_tail && j == Tk - 1 && threadIdx.x == 128) mbar_arrive(bar_v_tail);
       mbar_wait(bar_s_full + 8 * i, j & 1);
       if (tw) tr(1 + i, j, 0);
       tc_fence_after();

@@ -414,6 +414,9 @@ __device__ __forceinline__ uint32_t pack_bf162(float lo, float hi) {
 __device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
   asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
+__device__ __forceinline__ void st_shared_u16(uint32_t addr, uint16_t a) {
+  asm volatile("st.shared.u16 [%0], %1;" ::"r"(addr), "h"(a) : "memory");
+}
 __device__ __forceinline__ float fast_exp2(float x) {
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));

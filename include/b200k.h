@@ -104,7 +104,8 @@ int b200k_ffpa_fwd_f16(const void* Q, const void* K, const void* V, void* O, int
  *   dtype      B200K_F16 or B200K_BF16 (Q, K, V, O and the P operand; statistics and accumulators stay fp32)
  *   causal     != 0: query row r attends keys <= r; KV tiles above the diagonal are skipped, not masked
  *   seqlens_k  NULL, or int32 device array [B]: keys >= seqlens_k[b] are masked for batch b (key-padding mask of the
- *              padded [B,H,N,D] layout; 1 <= seqlens_k[b] <= N; every query row is still computed)
+ *              padded [B,H,N,D] layout; 1 <= seqlens_k[b] <= N; every query row is still computed).  K and V past
+ *              seqlens_k[b] are never used and may be uninitialised.
  * b200k_fa2_fwd_f16(...) == b200k_fa2_fwd(..., B200K_F16, 0, NULL, ...). */
 int b200k_fa2_fwd(const void* Q, const void* K, const void* V, void* O, int64_t B, int64_t H, int64_t N, int64_t D,
                   float scale, int v_is_dn, int dtype, int causal, const int* seqlens_k, int variant, void* stream);
